@@ -3,7 +3,7 @@
 precision, grad_clip=1.0), measured through the ``Stoke`` API.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--oss]
-                    [--workload resnet50|bert|allreduce_sweep]
+                    [--workload resnet50|bert|allreduce_sweep] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One step = ``out = s.model(x); l = s.loss(out, y); s.backward(l); s.step()`` on one synthetic batch per GPU.
@@ -21,6 +21,13 @@ Prints ONE JSON line on rank 0:
 ``--impl reference`` times the reference's CPU implementation alone: the UNMODIFIED reference package when
 ``oracle/_ref`` holds it (``oracle/build_ref.py``; ``kind: "reference"``), else the pinned port (``kind: "port"``).
 ``--workload bert`` is BASELINE configs[3] (BERT-base, length-bucketed sampler), ``--workload allreduce_sweep`` configs[4].
+``--dump-outputs DIR`` writes, on rank 0, what the last step of the timed resident loop returned to its caller, so that two
+builds can be compared output for output (the inputs depend only on the arguments): ``output.npy`` (the model's output,
+float32), ``loss.npy`` (the loss, float64) and ``params.npy`` (the updated model parameters in registration order, float32;
+a fixed sample of DUMP_PARAMS of them, drawn with seed 0, when there are more).  A dump run makes cuDNN use deterministic
+algorithms instead of autotuning, so that repeating it reproduces the dump; take timings from runs without the flag.  On
+one B200 two resnet50 dumps agreed bit for bit; two bert dumps did not (its attention backward is not deterministic):
+with ``--steps 5 --warmup 3`` their outputs differed by 1.3e-2 and their parameters by 5e-4 in relative L2.
 """
 import argparse
 import json
@@ -39,6 +46,8 @@ WORKLOAD = "resnet50_synthetic_3x224x224_ddp_bf16_adam_clipnorm1.0"
 ADAM = {"lr": 1e-3}
 CPU_SAMPLE_BATCH = 16
 RESNET50_PARAMS = 25_557_032
+DUMP_PARAMS = 1 << 22
+DUMP_MAX_BYTES = 64 << 20
 
 
 def parse():
@@ -55,7 +64,14 @@ def parse():
     ap.add_argument("--ncu-step", action="store_true",
                     help="profiling helper: warm up, then run ONE step between cudaProfilerStart/Stop and exit "
                          "(use with ncu --profile-from-start off); prints no bench line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (resnet50 and bert workloads)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "allreduce_sweep"):
+        ap.error("--dump-outputs needs --impl b200 and the resnet50 or bert workload")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -250,8 +266,29 @@ def parity_check(eng, rank, world):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+def dump_outputs(directory, s, last_step):
+    """Writes the model output and loss of the last resident step and the model parameters after it (see --dump-outputs)."""
+    import numpy as np
+    import torch
+
+    params = torch.cat([p.detach().reshape(-1).float() for p in s.model_access.parameters()])
+    if params.numel() > DUMP_PARAMS:
+        pick = np.sort(np.random.default_rng(0).choice(params.numel(), DUMP_PARAMS, replace=False))
+        params = params[torch.from_numpy(pick).to(params.device)]
+    arrays = {"output": last_step["output"].detach().float().cpu().numpy(),
+              "loss": last_step["loss"].detach().double().reshape(1).cpu().numpy(),
+              "params": params.cpu().numpy()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES} byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def build_workload(args, sb, torch, local_rank, world, rank):
-    """(stoke object, resident step fn, e2e step fn, per-GPU batch, h2d bytes per step, workload name, extras)."""
+    """(stoke object, resident step fn, e2e step fn, per-GPU batch, h2d bytes per step, workload name, extras, last_step).
+    ``last_step`` holds the model output and loss of the most recent resident step (references only: no copy, no sync)."""
     from stoke_b200 import synthetic
     from stoke_b200.data import DevicePrefetcher
 
@@ -269,9 +306,12 @@ def build_workload(args, sb, torch, local_rank, world, rank):
         x_host = x_host.contiguous(memory_format=torch.channels_last).pin_memory()
         y_host = y_host.pin_memory()
         x_dev, y_dev = x_host.to(dev), y_host.to(dev)
+        last_step = {}
 
         def step_resident():
-            s.backward(s.loss(s.model(x_dev), y_dev))
+            last_step["output"] = s.model(x_dev)
+            last_step["loss"] = s.loss(last_step["output"], y_dev)
+            s.backward(last_step["loss"])
             s.step()
 
         def host_batches():
@@ -290,7 +330,7 @@ def build_workload(args, sb, torch, local_rank, world, rank):
             return last
 
         h2d = x_host.numel() * x_host.element_size() + y_host.numel() * y_host.element_size()
-        return s, step_resident, step_e2e, batch, h2d, WORKLOAD + ("_oss" if common["fairscale_oss"] else ""), {}
+        return s, step_resident, step_e2e, batch, h2d, WORKLOAD + ("_oss" if common["fairscale_oss"] else ""), {}, last_step
 
     # ---- configs[3]: BERT-base, length-bucketed batches from BucketedDistributedSampler ----
     import numpy as np
@@ -330,11 +370,14 @@ def build_workload(args, sb, torch, local_rank, world, rank):
     pool = firsts + rest
     resident = [tuple(t.to(dev) for t in b) for b in pool]
     counter = {"i": 0}
+    last_step = {}
 
     def step_resident():
         ids, mask, y = resident[counter["i"] % len(resident)]
         counter["i"] += 1
-        s.backward(s.loss(s.model(input_ids=ids, attention_mask=mask).logits, y))
+        last_step["output"] = s.model(input_ids=ids, attention_mask=mask).logits
+        last_step["loss"] = s.loss(last_step["output"], y)
+        s.backward(last_step["loss"])
         s.step()
 
     def host_batches():
@@ -355,7 +398,8 @@ def build_workload(args, sb, torch, local_rank, world, rank):
     h2d = int(sum(sum(t.numel() * t.element_size() for t in b) for b in pool) / len(pool))
     extras = {"_distinct_shapes": len(seen), "sampler_setup_ms": sampler_ms, "dataset_items": n_items, "buckets": 16,
               "mean_padded_len": float(sum(b[0].shape[1] for b in pool) / len(pool))}
-    return s, step_resident, step_e2e, batch, h2d, "bert_base_synthetic_bucketed_sampler_ddp_bf16_adamw_clipnorm1.0", extras
+    return s, step_resident, step_e2e, batch, h2d, "bert_base_synthetic_bucketed_sampler_ddp_bf16_adamw_clipnorm1.0", extras, \
+        last_step
 
 
 def main():
@@ -397,9 +441,15 @@ def main():
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}: launch with torch.distributed.run")
     torch.cuda.set_device(local_rank)
     torch.backends.cudnn.benchmark = True
+    if args.dump_outputs:
+        # the autotuner's choice and cuDNN's non-deterministic algorithms change the last bits from run to run, and Adam
+        # on the repeated batch amplifies them into different weights: a dump run uses fixed, deterministic algorithms
+        torch.backends.cudnn.benchmark = False
+        torch.backends.cudnn.deterministic = True
     dev = torch.device("cuda", local_rank)
 
-    s, step_resident, step_e2e, batch, h2d_bytes, workload, extras = build_workload(args, sb, torch, local_rank, world, rank)
+    s, step_resident, step_e2e, batch, h2d_bytes, workload, extras, last_step = build_workload(args, sb, torch, local_rank,
+                                                                                               world, rank)
     eng = s.engine
     path = s.optimizer.path
 
@@ -458,6 +508,8 @@ def main():
     k1_dev_ms, k1_dev_n, k1_zero_ms = eng.profile_read_k1_device()
     k2_dev_ms, k2_dev_n = eng.profile_read_k2_device()
     eng.profile(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, s, last_step)
 
     # ---- timed region 2: end to end (H2D of the batch + D2H of the loss inside the timed region) ----
     for _ in range(2):

@@ -30,13 +30,3 @@ def pytest_collection_modifyitems(config, items):
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
-
-
-@pytest.fixture(scope="session")
-def reference_stoke():
-    """The unmodified reference package, or skip when /root/reference is absent (GPU box)."""
-    import ref_shim
-
-    if not ref_shim.reference_available():
-        pytest.skip("reference tree not present")
-    return ref_shim.import_reference()

@@ -1,9 +1,10 @@
 """CPU tests of the facade's own bookkeeping (accumulation cadence, loss tracking, EMA, wrap order) with a recording test
 double in place of the runner -- the engine itself needs a GPU.  The expected values are the unmodified reference's
-(tests/golden/cfg1_*.npz: counter trace) and, when /root/reference is present, a live side-by-side run."""
-import io
+(tests/golden/cfg1_*.npz: counter trace; tests/golden/reference_traces.json: per-micro-step loss bookkeeping)."""
+import hashlib
+import json
 import os
-from contextlib import nullcontext, redirect_stdout
+from contextlib import nullcontext
 
 import numpy as np
 import pytest
@@ -91,25 +92,26 @@ def test_counter_trace_and_weights_match_reference_fixture(fake_stoke, golden_di
     assert per_step[:6] == ["no_sync", "backward", "backward", "clip", "step", "no_sync"]
 
 
-def test_loss_tracking_matches_live_reference(fake_stoke, reference_stoke):
-    ref = reference_stoke
-    m_ref, m_new = synthetic.basic_nn(2), synthetic.basic_nn(2)
-    with redirect_stdout(io.StringIO()):
-        s_ref = ref.Stoke(model=m_ref, optimizer=ref.StokeOptimizer(optimizer=torch.optim.Adam,
-                          optimizer_kwargs=synthetic.CFG1_ADAM), loss=torch.nn.BCEWithLogitsLoss(),
-                          batch_size_per_device=32, grad_accum_steps=3, gpu=False, verbose=False, ema_weight=0.3)
-    s_new, _ = fake_stoke(m_new, 3)
-    s_new._ema_weight = 0.3
-    for x, y in synthetic.cfg1_batches(20, seed=9):
-        for s in (s_ref, s_new):
-            l = s.loss(s.model(x), y)
-            s.backward(l)
-            s.step()
-        assert s_ref.step_loss == s_new.step_loss
-        assert s_ref.ema_loss == s_new.ema_loss
-        assert s_ref._agg_loss == s_new._agg_loss
-        assert (s_ref._grad_accum_counter, s_ref._backward_steps, s_ref._optimizer_steps) == (
-            s_new._grad_accum_counter, s_new._backward_steps, s_new._optimizer_steps)
+def _reference_trace(golden_dir, name):
+    with open(os.path.join(golden_dir, "reference_traces.json")) as f:
+        return json.load(f)[name]
+
+
+def test_loss_tracking_matches_live_reference(fake_stoke, golden_dir):
+    rec = _reference_trace(golden_dir, "adam_accum3_ema03")
+    m_new = synthetic.basic_nn(rec["model_seed"])
+    s_new, _ = fake_stoke(m_new, rec["accum"])
+    s_new._ema_weight = rec["ema_weight"]
+    batches = list(synthetic.cfg1_batches(rec["batches"], seed=rec["batch_seed"]))
+    assert len(batches) == len(rec["steps"])
+    for (x, y), ref in zip(batches, rec["steps"]):
+        l = s_new.loss(s_new.model(x), y)
+        s_new.backward(l)
+        s_new.step()
+        assert ref["step_loss"] == s_new.step_loss
+        assert ref["ema_loss"] == s_new.ema_loss
+        assert ref["agg_loss"] == s_new._agg_loss
+        assert ref["counters"] == [s_new._grad_accum_counter, s_new._backward_steps, s_new._optimizer_steps]
     m_new.eval()
     x, y = next(iter(synthetic.cfg1_batches(1)))
     assert torch.equal(s_new.loss(s_new.model(x), y), torch.nn.BCEWithLogitsLoss()(m_new(x), y))  # no /accum in eval
@@ -148,32 +150,28 @@ def test_exports_cover_reference_names():
         assert hasattr(sb, name)
 
 
-def test_multiple_losses_bookkeeping_matches_live_reference(fake_stoke, reference_stoke):
+def test_multiple_losses_bookkeeping_matches_live_reference(fake_stoke, golden_dir):
     """List / tuple of loss callables (stoke/stoke.py:889-901): per-loss synced values, aggregated sums, EMA, the division by
-    grad_accum, and the retain_graph backward over the list -- side by side with the unmodified reference on CPU."""
-    ref = reference_stoke
+    grad_accum, and the retain_graph backward over the list -- against the unmodified reference's run on CPU."""
+    rec = _reference_trace(golden_dir, "multiple_losses")
 
     def losses():
         return [torch.nn.BCEWithLogitsLoss(), lambda out, y: ((out - y) ** 2).mean()]
 
-    m_ref, m_new = synthetic.basic_nn(8), synthetic.basic_nn(8)
-    with redirect_stdout(io.StringIO()):
-        s_ref = ref.Stoke(model=m_ref, optimizer=ref.StokeOptimizer(optimizer=torch.optim.Adam,
-                          optimizer_kwargs=synthetic.CFG1_ADAM), loss=losses(), batch_size_per_device=32,
-                          grad_accum_steps=2, gpu=False, verbose=False)
-    s_new, _ = fake_stoke(m_new, 2, loss=losses())
-    for x, y in synthetic.cfg1_batches(9, seed=4):
-        for s in (s_ref, s_new):
-            l = s.loss(s.model(x), y)
-            assert isinstance(l, list) and len(l) == 2
-            s.backward(l)
-            s.step()
-        assert s_ref.step_loss == s_new.step_loss
-        assert s_ref._agg_loss == s_new._agg_loss
-        assert s_ref.ema_loss == s_new.ema_loss
-    a = torch.cat([p.detach().reshape(-1) for p in m_ref.parameters()])
-    b = torch.cat([p.detach().reshape(-1) for p in m_new.parameters()])
-    assert torch.equal(a, b)
+    m_new = synthetic.basic_nn(rec["model_seed"])
+    s_new, _ = fake_stoke(m_new, rec["accum"], loss=losses())
+    batches = list(synthetic.cfg1_batches(rec["batches"], seed=rec["batch_seed"]))
+    assert len(batches) == len(rec["steps"])
+    for (x, y), ref in zip(batches, rec["steps"]):
+        l = s_new.loss(s_new.model(x), y)
+        assert isinstance(l, list) and len(l) == 2
+        s_new.backward(l)
+        s_new.step()
+        assert ref["step_loss"] == s_new.step_loss
+        assert ref["agg_loss"] == s_new._agg_loss
+        assert ref["ema_loss"] == s_new.ema_loss
+    b = torch.cat([p.detach().reshape(-1) for p in m_new.parameters()]).numpy()
+    assert hashlib.sha256(np.ascontiguousarray(b, dtype="<f4").tobytes()).hexdigest() == rec["final_sha256"]
 
 
 def test_lazy_loss_queue_folds_in_order(fake_stoke):
