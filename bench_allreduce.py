@@ -181,17 +181,6 @@ def main(argv=None):
         row["ours_ldg_fp32_us"] = t * 1e3
         row["ours_ldg_fp32_busbw"] = (world - 1) / world * n * 6 / (t * 1e-3) / 1e9
         eng.set_k1_algo("bulk")
-        if S <= (1 << 20):
-            # small buckets: the one-shot form (every rank reduces the whole bucket itself; default up to 256 KiB) against the
-            # two-shot form forced on the same size
-            default_kb = eng.option_get(_lib.OPT_K1_ONE_SHOT_KB)
-            eng.option_set(_lib.OPT_K1_ONE_SHOT_KB, 0)
-            t = time_op(lambda: ours(O16, torch.bfloat16))
-            row["ours_2shot_bf16_us"] = t * 1e3
-            eng.option_set(_lib.OPT_K1_ONE_SHOT_KB, 1024)
-            t = time_op(lambda: ours(O16, torch.bfloat16))
-            row["ours_1shot_bf16_us"] = t * 1e3
-            eng.option_set(_lib.OPT_K1_ONE_SHOT_KB, default_kb)
         if have_nvls:
             # multimem flavour: the NVSwitch reduces (multimem.ld_reduce) and replicates (multimem.st)
             eng.set_k1_algo("nvls")

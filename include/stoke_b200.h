@@ -151,17 +151,12 @@ int stk_comm_poll(stk_ctx* ctx);
  *     output buffers are multicast-bound and there is no local accumulator, otherwise the call falls back to 1 / 0.
  *     16-bit sums are rounded to the input type by the switch (fp32 accumulation inside it) -- NCCL's NVLS numerics.
  * STK_OPT_MEM_MODE: 0 = ipc, 1 = vmm (see stk_mem_alloc_shared).  STK_OPT_K1_MAX_BLOCKS: grid bound of the cross-rank
- * K1 (default: one block per SM); smaller grids leave SMs to a concurrently running backward. */
+ * K1 (0, the default: one block per SM).  STK_OPT_NVLS_MAX_BLOCKS: grid bound of the multimem flavour alone (0, the
+ * default: 8 blocks below 128 MiB of input, 16 above).  The two grid bounds exist for bandwidth studies.
+ * Cross-rank kernels always use cooperative launches: their blocks spin on the peers' blocks and must be co-resident. */
 #define STK_OPT_MEM_MODE 2
 #define STK_OPT_K1_MAX_BLOCKS 3
-#define STK_OPT_COOP_LAUNCH 4   /* 1 (default): cross-rank kernels use cooperative launches (co-residency enforced) */
-#define STK_OPT_NVLS_MAX_BLOCKS 5 /* grid bound of the multimem flavour alone (0: same as STK_OPT_K1_MAX_BLOCKS) */
-#define STK_OPT_K2_AG_MC 6      /* 1: the sharded step publishes its shard with multimem.st when the parameter buffer is bound */
-#define STK_OPT_K1_ONE_SHOT_KB 7 /* all-reduce buckets of at most this many KiB of input take the ONE-SHOT form: every rank reads
-                                    the whole bucket from all W peers and reduces all of it itself (W x the loads, but no peer
-                                    stores, no store-completion fence, no cross-rank partial exchange: the small-message
-                                    latency path).  Default 0 = always two-shot (the one-shot form measured 3-5 us SLOWER at W = 2:
-                                    21.5 vs 18.2 us at 64 KiB; not measured at W = 8).  Same results (rank-order fp32 sums). */
+#define STK_OPT_NVLS_MAX_BLOCKS 5
 int stk_option_set(stk_ctx* ctx, int key, int value);
 int stk_option_get(stk_ctx* ctx, int key, int* value);
 

@@ -16,7 +16,7 @@ NORM_NONE, NORM_L2, NORM_INF, NORM_P = 0, 1, 2, 3
 CLIP_NONE, CLIP_NORM, CLIP_VALUE = 0, 1, 2
 OPT_ADAM, OPT_ADAMW, OPT_SGD = 0, 1, 2
 RF_FINAL, RF_ZERO_INPUT, RF_UNSCALE = 1, 2, 4
-OPT_K1_ALGO, OPT_MEM_MODE, OPT_K1_MAX_BLOCKS, OPT_COOP_LAUNCH, OPT_NVLS_MAX_BLOCKS, OPT_K2_AG_MC, OPT_K1_ONE_SHOT_KB = 1, 2, 3, 4, 5, 6, 7
+OPT_K1_ALGO, OPT_MEM_MODE, OPT_K1_MAX_BLOCKS, OPT_NVLS_MAX_BLOCKS = 1, 2, 3, 5
 K1_ALGO_LDG, K1_ALGO_BULK, K1_ALGO_NVLS = 0, 1, 2
 MAX_GROUPS, MAX_SEGMENTS, LOSS_RING = 8, 64, 256
 ERR_INVALID, ERR_CUDA, ERR_STATE, ERR_PEER, ERR_UNSUPPORTED = -1, -2, -3, -4, -5

@@ -173,10 +173,7 @@ int stk_bcast(stk_ctx* c, void* const* ptrs, size_t bytes, int root, void* strea
   cfg.blockDim = dim3(512);
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeCooperative;
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = c->coop_launch ? 1 : 0;
+  coop_attr(cfg, attr);
   const uint4* src = reinterpret_cast<const uint4*>(ptrs[root]);
   uint4* dst = reinterpret_cast<uint4*>(ptrs[c->rank]);
   uint32_t epoch = ++c->blk_epoch;

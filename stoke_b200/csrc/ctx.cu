@@ -37,7 +37,7 @@ int stk_grow_partials(stk_ctx* c, size_t blocks, cudaStream_t s) {
 
 extern "C" {
 
-int stk_version(void) { return 200; }
+int stk_version(void) { return 201; }
 
 const char* stk_last_error(stk_ctx* ctx) {
   if (ctx && !ctx->err.empty()) return ctx->err.c_str();
@@ -63,11 +63,6 @@ int stk_ctx_create(int rank, int world, int device, unsigned flags, stk_ctx** ou
   c->sm_count = prop.multiProcessorCount;
   if (const char* algo = std::getenv("STK_K1_ALGO"))
     c->k1_algo = (std::strcmp(algo, "nvls") == 0) ? 2 : (std::strcmp(algo, "bulk") == 0) ? 1 : 0;
-  if (const char* v = std::getenv("STK_K1_MAX_BLOCKS")) c->k1_max_blocks = std::atoi(v);
-  if (const char* v = std::getenv("STK_COOP_LAUNCH")) c->coop_launch = std::atoi(v) != 0;
-  if (const char* v = std::getenv("STK_NVLS_MAX_BLOCKS")) c->nvls_max_blocks = std::atoi(v);
-  if (const char* v = std::getenv("STK_K2_AG")) c->k2_ag_mc = std::strcmp(v, "mc") == 0;
-  if (const char* v = std::getenv("STK_K1_ONE_SHOT_KB")) c->one_shot_bytes = size_t(std::max(0, std::atoi(v))) << 10;
   // memory back end: VMM (needed for NVLS multicast) when there are peers and the driver supports it
   bool mc = false;
   const bool vmm = stk_vmm_available(device, &mc);
@@ -434,19 +429,9 @@ int stk_option_set(stk_ctx* c, int key, int value) {
       STK_REQUIRE(c, value >= 0 && value <= stk::kMaxReduceBlocks, "stk_option_set: K1 max blocks out of range");
       c->k1_max_blocks = value;
       return STK_OK;
-    case STK_OPT_COOP_LAUNCH:
-      c->coop_launch = value != 0;
-      return STK_OK;
     case STK_OPT_NVLS_MAX_BLOCKS:
       STK_REQUIRE(c, value >= 0 && value <= stk::kMaxReduceBlocks, "stk_option_set: NVLS max blocks out of range");
       c->nvls_max_blocks = value;
-      return STK_OK;
-    case STK_OPT_K2_AG_MC:
-      c->k2_ag_mc = value != 0;
-      return STK_OK;
-    case STK_OPT_K1_ONE_SHOT_KB:
-      STK_REQUIRE(c, value >= 0, "stk_option_set: one-shot threshold must be >= 0 KiB");
-      c->one_shot_bytes = size_t(value) << 10;
       return STK_OK;
     default:
       return stk_fail(c, STK_ERR_INVALID, "stk_option_set: unknown key");
@@ -460,10 +445,7 @@ int stk_option_get(stk_ctx* c, int key, int* value) {
     case STK_OPT_K1_ALGO: *value = c->k1_algo; return STK_OK;
     case STK_OPT_MEM_MODE: *value = c->mem_mode; return STK_OK;
     case STK_OPT_K1_MAX_BLOCKS: *value = c->k1_max_blocks; return STK_OK;
-    case STK_OPT_COOP_LAUNCH: *value = c->coop_launch; return STK_OK;
     case STK_OPT_NVLS_MAX_BLOCKS: *value = c->nvls_max_blocks; return STK_OK;
-    case STK_OPT_K2_AG_MC: *value = c->k2_ag_mc; return STK_OK;
-    case STK_OPT_K1_ONE_SHOT_KB: *value = (int)(c->one_shot_bytes >> 10); return STK_OK;
     default: return stk_fail(c, STK_ERR_INVALID, "stk_option_get: unknown key");
   }
 }

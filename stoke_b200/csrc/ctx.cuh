@@ -57,11 +57,7 @@ struct stk_ctx {
   uint32_t aux_epoch[4] = {0, 0, 0, 0};
   int k1_algo = 1;              // cross-rank K1 flavour: 0 = register-staged loads, 1 = bulk-async (default), 2 = multimem (NVLS)
   int k1_max_blocks = 0;        // 0: one block per SM
-  int coop_launch = 1;
   int nvls_max_blocks = 0;      // grid bound of the multimem flavour (0: like the other flavours)
-  size_t one_shot_bytes = 0;    // all-reduce buckets up to this many input bytes take the one-shot form (0 = never, the default:
-                                // measured slower than the two-shot form at W = 2, profiles/allreduce_r02.md)
-  int k2_ag_mc = 0;             // sharded step publishes its shard with multimem.st (one store replicated by the switch)
   // device state
   std::vector<StepState> states;      // [0] is created with the context
   int cur_state = 0;
@@ -148,6 +144,15 @@ static inline int blocks_per_sm(stk_ctx* c, K kernel, int threads, size_t smem =
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
   c->occupancy[key] = per_sm;
   return per_sm;
+}
+
+// Every cross-rank kernel spins on its peers' blocks, so all of its blocks must be co-resident: the cooperative attribute
+// makes the launch fail instead of deadlocking when the grid does not fit.  `attr` must outlive the launch call.
+inline void coop_attr(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr) {
+  attr[0].id = cudaLaunchAttributeCooperative;
+  attr[0].val.cooperative = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
 }
 
 struct DeviceGuard {

@@ -157,7 +157,7 @@ static cudaError_t launch_bulk_t(stk_ctx* c, const ReduceParams& p, int grid, cu
   cfg.dynamicSmemBytes = smem;
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
-  coop_attr(c, cfg, attr);
+  coop_attr(cfg, attr);
   ProfScope prof(c, 0, s);
 #define STK_BULK(WT)                                                                                              \
   {                                                                                                               \

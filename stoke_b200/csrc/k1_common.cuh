@@ -24,7 +24,6 @@ struct ReduceParams {
   float mul;
   float norm_p;
   int rank, world, n_dst;
-  int one_shot;        // small all-reduce: every rank sums the WHOLE bucket from all peers itself (no peer stores, no partial exchange)
   int norm_kind;
   uint32_t flags;
   uint32_t epoch, aux_epoch;
@@ -110,13 +109,12 @@ __device__ __forceinline__ void reduce_tail(const ReduceParams& p, float part, b
     any_bad = __any_sync(0xffffffffu, threadIdx.x < nwarp && s_bad[threadIdx.x] != 0);
   }
 
-  const bool exchange = W > 1 && !p.one_shot;  // one-shot: every rank reduced everything itself, its own partials are global
   if (W > 1) {
     // Publish this block's (norm partial, inf flag) to every rank BEFORE signalling the end barrier: the same thread then
     // does fence.sys + st.release of the flag, so whoever sees the flag sees the partial.  Every rank later sums all
     // W x grid partials in the same (rank, block) order -> bit-identical totals everywhere, with no third cross-GPU
     // round trip after the data phase.
-    if (exchange && threadIdx.x < (unsigned)W) {
+    if (threadIdx.x < (unsigned)W) {
       RankScalars* slot = &p.pads.p[threadIdx.x]->blk_scal[p.rank][blockIdx.x];
       st_relaxed_sys_f32(&slot->norm_partial, blk);
       st_relaxed_sys_u32(&slot->found_inf, any_bad);
@@ -132,8 +130,7 @@ __device__ __forceinline__ void reduce_tail(const ReduceParams& p, float part, b
     // Zero the LOCAL gradient bucket inside the kernel (no separate memset between backward and step).  Block b may only
     // clear what the peers' blocks b have finished reading -- exactly this block's own index pattern, replicated in every
     // shard: shard q of my bucket is read by rank q's block b at the same offsets, and that block has passed the end barrier.
-    const int Q = p.one_shot ? 1 : W;  // one-shot: the peers' blocks b read this block's pattern over the whole bucket
-    for (int q = 0; q < Q; ++q) {
+    for (int q = 0; q < W; ++q) {
       const size_t qb = p.vec_per_shard * q;
       size_t qe = qb + p.vec_per_shard;
       if (qe > p.vec_total) qe = p.vec_total;
@@ -153,7 +150,7 @@ __device__ __forceinline__ void reduce_tail(const ReduceParams& p, float part, b
   const unsigned lane = threadIdx.x;
   const bool mx = p.norm_kind == STK_NORM_INF;
 
-  if (exchange) {
+  if (W > 1) {
     // ---- cross-rank flavour: plain ticket over the (<= SM count) co-resident blocks ----
     unsigned last = 0;
     if (lane == 0) {
@@ -270,12 +267,5 @@ __device__ __forceinline__ void reduce_tail(const ReduceParams& p, float part, b
 cudaError_t launch_reduce_bulk(stk_ctx* c, const ReduceParams& p, int grad_dtype, int out_dtype, int grid, cudaStream_t s);
 // k1_nvls.cu: multimem (NVSwitch in-network reduction) flavour; cudaErrorNotSupported -> next flavour
 cudaError_t launch_reduce_nvls(stk_ctx* c, const ReduceParams& p, int grad_dtype, int out_dtype, int grid, cudaStream_t s);
-
-inline void coop_attr(stk_ctx* c, cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr) {
-  attr[0].id = cudaLaunchAttributeCooperative;
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = c->coop_launch ? 1 : 0;
-}
 
 }  // namespace stk

@@ -9,8 +9,6 @@
 //                  HBM instead of 8 + 30 (no fp32 main-grad round trip).
 //   k_grad_scale : grad *= clip coefficient, or clamp (clip_grad_norm_'s scaling pass / clip_grad_value_,
 //                  torch/nn/utils/clip_grad.py) for optimizers the fused step does not cover.
-#include <cstdlib>
-
 #include "k1_common.cuh"
 
 namespace stk {
@@ -20,7 +18,9 @@ __device__ __forceinline__ uint64_t policy_evict_last() {
   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
-__device__ __forceinline__ uint4 ld16_keep(const void* p, uint64_t pol) {  // bypass L1, keep in L2
+// Bypass L1, keep in L2: the fused step's second read of a bucket that fits L2 then hits (measured -4 us on K2 at
+// ResNet-50 size, profiles/kernels_r02.md).
+__device__ __forceinline__ uint4 ld16_keep(const void* p, uint64_t pol) {
   uint4 v;
   asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.u32 {%0,%1,%2,%3}, [%4], %5;"
                : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
@@ -35,8 +35,6 @@ struct NormParams {
   float mul, norm_p;
   int norm_kind;
   uint32_t flags;
-  int keep_l2;       // 1 (default; STK_NORM_L2_KEEP=0 disables): loads carry an L2 evict_last policy -- the fused step's second
-                     // read of a bucket that fits L2 then hits: measured -4 us on K2 at ResNet-50 size (profiles/kernels_r02.md)
   stk_scaler_state_t* scaler;
   StepAccum* accum;
   float* blk_partial;
@@ -47,10 +45,10 @@ struct RawVec;  // the raw words of one 8-element vector (kept packed until use:
 template <>
 struct RawVec<STK_F32> {
   uint4 a, b;
-  __device__ void load(const void* base, size_t v, uint64_t pol, bool keep) {
+  __device__ void load(const void* base, size_t v, uint64_t pol) {
     const uint4* q = reinterpret_cast<const uint4*>(base) + 2 * v;
-    a = keep ? ld16_keep(q, pol) : ld_stream16(q);
-    b = keep ? ld16_keep(q + 1, pol) : ld_stream16(q + 1);
+    a = ld16_keep(q, pol);
+    b = ld16_keep(q + 1, pol);
   }
   __device__ void unpack(float (&f)[8]) const {
     f[0] = __uint_as_float(a.x); f[1] = __uint_as_float(a.y); f[2] = __uint_as_float(a.z); f[3] = __uint_as_float(a.w);
@@ -60,9 +58,8 @@ struct RawVec<STK_F32> {
 template <int DT16>
 struct RawVec16 {
   uint4 u;
-  __device__ void load(const void* base, size_t v, uint64_t pol, bool keep) {
-    const uint4* q = reinterpret_cast<const uint4*>(base) + v;
-    u = keep ? ld16_keep(q, pol) : ld_stream16(q);
+  __device__ void load(const void* base, size_t v, uint64_t pol) {
+    u = ld16_keep(reinterpret_cast<const uint4*>(base) + v, pol);
   }
   __device__ void unpack(float (&f)[8]) const {
     const uint32_t w4[4] = {u.x, u.y, u.z, u.w};
@@ -99,7 +96,7 @@ __global__ void __launch_bounds__(kNormThreads) k_grad_norm(const NormParams p) 
 #pragma unroll
   for (int u = 0; u < kNormUnroll; ++u) {
     const size_t v = t0 + size_t(u) * kNormThreads + threadIdx.x;
-    if (v < p.nvec) raw[u].load(p.grad, v, pol, p.keep_l2 != 0);
+    if (v < p.nvec) raw[u].load(p.grad, v, pol);
   }
 #pragma unroll
   for (int u = 0; u < kNormUnroll; ++u) {
@@ -205,14 +202,6 @@ int stk_grad_norm(stk_ctx* c, const void* grad, int grad_dtype, const float* acc
   p.norm_p = (float)norm_p;
   p.norm_kind = norm_kind;
   p.flags = flags;
-  {
-    static int keep = -1;
-    if (keep < 0) {
-      const char* e = std::getenv("STK_NORM_L2_KEEP");
-      keep = e ? std::atoi(e) : 1;
-    }
-    p.keep_l2 = keep;
-  }
   p.scaler = c->scaler_dev;
   p.accum = c->accum_dev;
   const size_t tile = size_t(kNormThreads) * kNormUnroll;

@@ -130,7 +130,7 @@ static cudaError_t launch_nvls_t(stk_ctx* c, const ReduceParams& p, int grid, cu
   cfg.blockDim = dim3(kNvlsThreads);
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
-  coop_attr(c, cfg, attr);
+  coop_attr(cfg, attr);
   ProfScope prof(c, 0, s);
   // small shards: one round per thread is enough; large shards: 4 independent switch requests in flight per thread
   const size_t shard_vecs = p.vec_end - p.vec_begin;

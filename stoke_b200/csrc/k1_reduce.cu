@@ -144,8 +144,7 @@ static cudaError_t launch_reduce(stk_ctx* c, const ReduceParams& p, int grid, bo
   cfg.blockDim = dim3(p.world == 1 ? 256 : 512);
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
-  coop_attr(c, cfg, attr);
-  if (!coop) cfg.numAttrs = 0;
+  if (coop) coop_attr(cfg, attr);
   ProfScope prof(c, 0, s);
   switch (p.world) {
     case 1: return cudaLaunchKernelEx(&cfg, k_grad_reduce<IN_DT, OUT_DT, 1>, p);
@@ -246,22 +245,10 @@ int stk_grad_reduce(stk_ctx* c, int mode, void* const* grad_ptrs, int grad_dtype
     p.grp_count = c->grp_count_dev;
   }
   const bool coop = W > 1;
-  // Small all-reduce buckets: one-shot form.  Every rank sums the whole bucket from all W peers in rank order (bit-identical
-  // on every rank by construction) and stores only locally; its own norm partials are already global.
-  const size_t in_bytes = n * (grad_dtype == STK_F32 ? 4 : 2);
-  if (coop && mode == STK_REDUCE_ALL && c->one_shot_bytes > 0 && in_bytes <= c->one_shot_bytes) {
-    p.one_shot = 1;
-    p.vec_begin = 0;
-    p.vec_end = p.vec_total;
-    p.vec_per_shard = p.vec_total;
-    p.n_dst = 1;
-    want = (p.vec_total + threads * U - 1) / (threads * U);
-    grid = (int)std::max<size_t>(1, std::min<size_t>(want, cap));
-  }
   if (coop && grid > kMaxReduceBlocks) grid = kMaxReduceBlocks;
 
   cudaError_t err = cudaErrorNotSupported;
-  if (coop && c->k1_algo == 2 && acc_ptrs == nullptr && !p.one_shot) {
+  if (coop && c->k1_algo == 2 && acc_ptrs == nullptr) {
     // multimem flavour: needs the multicast mappings of the gradient bucket and (all-reduce) of the output bucket
     p.grad_mc = stk_mc_lookup(c, grad_ptrs[c->rank]);
     p.out_mc = (mode == STK_REDUCE_ALL) ? stk_mc_lookup(c, out_ptrs[c->rank]) : nullptr;
@@ -277,7 +264,7 @@ int stk_grad_reduce(stk_ctx* c, int mode, void* const* grad_ptrs, int grad_dtype
     }
   }
   if (err == cudaSuccess) return STK_OK;
-  if (coop && c->k1_algo >= 1 && !p.one_shot) {
+  if (coop && c->k1_algo >= 1) {
     err = launch_reduce_bulk(c, p, grad_dtype, out_dtype, grid, s);
     if (err != cudaSuccess && err != cudaErrorNotSupported)
       return stk_fail(c, STK_ERR_CUDA, std::string("k_grad_reduce_bulk launch: ") + cudaGetErrorString(err));

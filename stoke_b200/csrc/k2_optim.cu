@@ -18,8 +18,6 @@
 // Arithmetic follows torch/optim/adam.py (_single_tensor_adam, the path torch takes on CPU -- the oracle) and
 // torch/optim/sgd.py (_single_tensor_sgd); the clip follows torch/nn/utils/clip_grad.py:165-174 (coef = max_norm /
 // (total_norm + 1e-6), clamped to 1) and :291-292 (clamp).
-#include <cstdlib>
-
 #include "k1_common.cuh"
 
 namespace stk {
@@ -41,7 +39,6 @@ struct OptimParams {
   const float* acc;     // RAW only
   size_t nvec;          // 8-float vector count of the local state
   PtrTable lp;          // low-precision / remote parameter destinations (bases; indexed globally)
-  void* lp_mc;          // multicast mapping of the parameter buffer: publish with ONE multimem.st instead of W peer stores
   unsigned long long* prof_ns;  // optional {ns between the barriers, launches} (block 0), nullptr when off
   int lp_world;         // 0: none
   int lp_rank_skip;     // lp dtype == f32 and destination == master's own buffer: skip that rank (aliased)
@@ -96,13 +93,6 @@ __device__ __forceinline__ void store_lp(const OptimParams& p, size_t gv, const 
     for (int k = 0; k < VPT; ++k)
       u[k] = make_uint4(pack_bf16(x[k][0], x[k][1]), pack_bf16(x[k][2], x[k][3]), pack_bf16(x[k][4], x[k][5]),
                         pack_bf16(x[k][6], x[k][7]));
-    if (p.lp_mc != nullptr) {
-      // the NVSwitch replicates the store into every rank's parameter buffer (this rank's own copy included)
-#pragma unroll
-      for (int k = 0; k < VPT; ++k)
-        if (k < nv) mm_st16(reinterpret_cast<uint4*>(p.lp_mc) + gv + k, u[k]);
-      return;
-    }
 #pragma unroll 1
     for (int d = 0; d < p.lp_world; ++d) {
       const int dst = p.lp_world == 1 ? 0 : (p.rank + d) % p.lp_world;
@@ -371,8 +361,7 @@ static cudaError_t launch_one(stk_ctx* c, K kernel, const OptimParams& p, bool p
   cfg.blockDim = dim3(256);
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
-  coop_attr(c, cfg, attr);
-  if (!persist) cfg.numAttrs = 0;
+  if (persist) coop_attr(cfg, attr);
   ProfScope prof(c, 1, s);
   return cudaLaunchKernelEx(&cfg, kernel, p);
 }
@@ -390,7 +379,7 @@ static cudaError_t launch_optim(stk_ctx* c, const OptimParams& p, int lp_dtype, 
   }
   if (p.cross_rank) {
     if (lp_dtype == STK_BF16) {
-      if (pair && p.lp_mc == nullptr) return launch_one(c, k_optim_step<KIND, STK_BF16, true, 2, STK_F32, false>, p, true, 2, s);
+      if (pair) return launch_one(c, k_optim_step<KIND, STK_BF16, true, 2, STK_F32, false>, p, true, 2, s);
       return launch_one(c, k_optim_step<KIND, STK_BF16, true, 1, STK_F32, false>, p, true, 1, s);
     }
     return launch_one(c, k_optim_step<KIND, STK_F32, true, 1, STK_F32, false>, p, true, 1, s);
@@ -470,8 +459,6 @@ int stk_optim_step_ex(stk_ctx* c, const stk_optim_args_t* a, void* stream) {
         static_cast<char*>(a->lp_ptrs[r]) + size_t(p.seg_global[0]) * 32 == reinterpret_cast<char*>(a->master))
       p.lp_rank_skip = r;
   }
-  p.lp_mc = nullptr;
-  if (cross && c->k2_ag_mc && a->lp_dtype != STK_F32) p.lp_mc = stk_mc_lookup(c, a->lp_ptrs[c->rank]);  // nullptr: not bound
   p.prof_ns = (cross && c->profiling) ? c->prof_ns_dev + 4 : nullptr;
   p.scaler = c->scaler_dev;
   p.pads = c->pads;
@@ -501,14 +488,6 @@ int stk_optim_step_ex(stk_ctx* c, const stk_optim_args_t* a, void* stream) {
     p.unscale = 1;
   }
 
-  {
-    static int pair_env = -1;   // STK_K2_PAIR=0: one vector per thread in the sharded step (16-byte peer stores, 3 blocks/SM)
-    if (pair_env < 0) {
-      const char* e = std::getenv("STK_K2_PAIR");
-      pair_env = e ? std::atoi(e) : 1;
-    }
-    if (!pair_env) pair_ok = false;
-  }
   cudaError_t err;
   const bool raw = a->grad_raw != 0;
   g_grid_nvec = cross ? (a->grid_n ? (a->grid_n + 7) / 8 : p.nvec) : 0;

@@ -267,15 +267,6 @@ class Engine:
         self._check(self.lib.stk_grad_scale(self.ctx, grad_ptr, n, clip_kind, max_norm, clip_value, self._stream()))
         self.launches += 1
 
-    def optim_step(self, hyper: _lib.OptimHyper, master_ptr: int, m_ptr: Optional[int], v_ptr: Optional[int],
-                   grad_ptr: int, n_local: int, lp_ptrs: Optional[Sequence[int]], lp_dtype: torch.dtype,
-                   lp_offset: int):
-        lp = _lib.ptr_array(lp_ptrs) if lp_ptrs is not None else None
-        self._check(self.lib.stk_optim_step(self.ctx, C.byref(hyper), master_ptr, m_ptr, v_ptr, grad_ptr, n_local, lp,
-                                            len(lp_ptrs) if lp_ptrs is not None else 0, _DT[lp_dtype], lp_offset,
-                                            self._stream()))
-        self.launches += 1
-
     def optim_step_ex(self, args: _lib.OptimArgs):
         self._check(self.lib.stk_optim_step_ex(self.ctx, C.byref(args), self._stream()))
         self.launches += 1
@@ -546,7 +537,6 @@ class GradPath:
         self._bucket_tabs = {}
         # ---- autograd hooks: per-bucket launches while backward runs, and unused-parameter detection ----
         self.overlap = bool(overlap) and W > 1 and len(self.buckets) > 1
-        self._overlap_blocks = int(os.environ.get("STK_K1_OVERLAP_BLOCKS", "0")) if self.overlap else 0
         self._comm_stream = torch.cuda.Stream(engine.device) if self.overlap else None
         self._hooks = []
         self._armed = False          # hooks launch K1 for this backward
@@ -639,10 +629,6 @@ class GradPath:
             self._comm_stream.wait_event(ev)
             stream = self._comm_stream
         e.state_select(self.state_id)
-        # grid of this launch: a function of the bucket index only (identical on every rank whatever launched it -- a hook or
-        # the flush after backward): every bucket but the last may run on a reduced grid so that it shares the SMs with backward
-        if self._overlap_blocks:
-            e.option_set(_lib.OPT_K1_MAX_BLOCKS, self._overlap_blocks if k < len(self.buckets) - 1 else 0)
         # pointer tables per bucket are built once (the hooks run on the autograd thread: keep them short)
         key = (k, has_acc)
         tabs = self._bucket_tabs.get(key)

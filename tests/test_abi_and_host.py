@@ -33,6 +33,19 @@ def test_header_symbols_exported(lib):
     assert lib.stk_version() >= 100
 
 
+def test_option_and_optimizer_constants_match_header():
+    """Every STK_OPT_<NAME> of the header (option keys are #defines, optimizer kinds an enum) is _lib.OPT_<NAME> with the
+    same value, and _lib has no OPT_ constant the header lacks."""
+    header = open(os.path.join(ROOT, "include", "stoke_b200.h")).read()
+    header = re.sub(r"/\*.*?\*/", "", header, flags=re.S)
+    pairs = re.findall(r"#define\s+STK_OPT_([A-Z0-9_]+)\s+(\d+)\b", header)
+    pairs += re.findall(r"\bSTK_OPT_([A-Z0-9_]+)\s*=\s*(\d+)\b", header)
+    declared = {name: int(v) for name, v in pairs}
+    assert len(declared) == len(pairs) and {"K1_ALGO", "ADAM"} <= set(declared)
+    mine = {k[len("OPT_"):]: v for k, v in vars(_lib).items() if k.startswith("OPT_")}
+    assert mine == declared, set(mine.items()) ^ set(declared.items())
+
+
 def test_struct_layouts_match_header():
     # sizes the C side static-asserts implicitly through use; guards against ctypes drift
     assert C.sizeof(_lib.ScalerState) == 48

@@ -291,6 +291,23 @@ def test_loss_sync_and_barrier_world1():
     eng.comm_check()
 
 
+def test_removed_option_keys_are_rejected():
+    """Keys 4 (non-cooperative launch), 6 (multimem.st publish) and 7 (one-shot all-reduce) no longer exist."""
+    from stoke_b200 import _lib
+    from stoke_b200.engine import get_engine
+
+    eng = get_engine(0)
+    for key in (4, 6, 7):
+        with pytest.raises(_lib.StokeB200Error) as e:
+            eng.option_set(key, 0)
+        assert e.value.code == _lib.ERR_INVALID
+        with pytest.raises(_lib.StokeB200Error) as e:
+            eng.option_get(key)
+        assert e.value.code == _lib.ERR_INVALID
+    for key in (_lib.OPT_K1_ALGO, _lib.OPT_MEM_MODE, _lib.OPT_K1_MAX_BLOCKS, _lib.OPT_NVLS_MAX_BLOCKS):
+        eng.option_get(key)
+
+
 def test_save_load_roundtrip(tmp_path):
     import stoke_b200 as sb
     from stoke_b200 import synthetic

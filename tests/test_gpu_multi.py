@@ -19,9 +19,7 @@ def _run(world, tmp_path, port, algo="ldg"):
            "127.0.0.1", "--master-port", str(port), os.path.join(ROOT, "tests", "mgpu_worker.py"), str(out)]
     # cross-rank K1 flavour: register-staged loads | bulk-async through smem | multimem (NVLS); tiny gradient buckets in the
     # Stoke-API section so that the per-bucket launches from autograd hooks are exercised on a small model
-    env = dict(os.environ, STK_K1_ALGO=algo, STK_BUCKET_MB="0.0005", STK_OVERLAP="on", STK_SPIN_TIMEOUT_S="30",
-               # the W = 2 ldg run also covers the (opt-in) one-shot small all-reduce
-               STK_K1_ONE_SHOT_KB="256" if (algo == "ldg" and world == 2) else "0")
+    env = dict(os.environ, STK_K1_ALGO=algo, STK_BUCKET_MB="0.0005", STK_OVERLAP="on", STK_SPIN_TIMEOUT_S="30")
     proc = subprocess.run(cmd, capture_output=True, text=True, timeout=420, env=env)
     assert proc.returncode == 0, proc.stdout[-4000:] + proc.stderr[-4000:]
     with open(out) as f:
